@@ -2,6 +2,7 @@
 """bench.py — the measured headline of this repository.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--mnk M_N_K] [--acc fp32|fp16] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Metric (BASELINE.json): HGEMM TFLOP/s, offline mode (back-to-back calls), per (M,N,K). One "step" is ONE
@@ -29,6 +30,11 @@ What is timed
           and a CUDA-event-timed back-to-back batch. Aggregate = sum of 2MNK over ALL shapes / max over ranks of the
           rank's summed device time, so it grows with N only if the sharding works.
 
+--dump-outputs DIR  writes C of the last timed step (rank 0) as DIR/c.npy, float32, so that two builds can be compared
+          output for output: the operands come from seeded generators, so the same arguments give the same inputs. An
+          output of more than DUMP_MAX_ELEMS entries is sampled at positions drawn with a fixed seed (sorted flat
+          row-major indices, the same for every run of the shape), which keeps the file under 64 MB.
+
 Multi-GPU: the path shards by problem (one GEMM per GPU, no collective on the data path; SURVEY §8e), so
 at N > 1 every rank runs the same per-GPU work ("scaling": "weak") and value is the sum over ranks.
 """
@@ -48,16 +54,25 @@ from pathlib import Path
 REPO = Path(__file__).resolve().parent
 sys.path.insert(0, str(REPO))
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 L2_BYTES = 126 * 1024 * 1024
 FALLBACK_TFLOPS, FALLBACK_HBM = 1590.0, 6650.0
+DUMP_MAX_ELEMS = 1 << 23        # 32 MiB of float32
+
+
+def positive_int(text: str) -> int:
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
 
 
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=2000)
+    p.add_argument("--steps", type=positive_int, default=2000, help="timed steps (GEMMs) of the headline value")
     p.add_argument("--warmup", type=int, default=20)
     p.add_argument("--mnk", type=str, default="4096_4096_4096")
     p.add_argument("--acc", type=str, default="fp32", choices=["fp32", "fp16"])
@@ -68,6 +83,9 @@ def parse_args():
     p.add_argument("--sweep", type=str, default="grid", help="'grid' (1001 shapes), 'none', or a comma list of M_N_K")
     p.add_argument("--sweep_ms", type=float, default=25.0, help="sampling budget per shape of the sweep leg")
     p.add_argument("--cpu_threads", type=int, default=0, help="threads of the CPU arms (0 = half the host's logical CPUs)")
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help=f"write C of the last timed step as DIR/c.npy (float32; at most {DUMP_MAX_ELEMS} entries, a fixed "
+                        "sample when C is larger)")
     return p.parse_args()
 
 
@@ -344,6 +362,16 @@ def run_sweep(args, capi, rank: int, world: int, dist) -> dict | None:
     }
 
 
+def output_sample(c: torch.Tensor) -> np.ndarray:
+    """``c`` as float32 on the host: whole up to DUMP_MAX_ELEMS entries, otherwise the entries at sorted flat indices
+    drawn with seed 0 (they depend on the shape only, so runs of the same shape are comparable entry for entry)."""
+    if c.numel() <= DUMP_MAX_ELEMS:
+        return c.float().cpu().numpy()
+    g = torch.Generator().manual_seed(0)
+    idx = torch.randint(c.numel(), (DUMP_MAX_ELEMS,), generator=g).unique()
+    return c.reshape(-1)[idx.to(c.device)].float().cpu().numpy()
+
+
 def main():
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -351,6 +379,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     m, n, k = (int(x) for x in args.mnk.split("_"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the GPU path's output; --impl reference has none")
         run_reference(args, m, n, k, rank, world)
         return 0
 
@@ -418,6 +448,8 @@ def main():
         launches = int(lt.item())
     flops_step = 2.0 * m * n * k
     value = flops_step * args.steps * world / (ms_total * 1e-3) * 1e-12
+    # taken now: the legs below run the same operand sets again
+    dump = output_sample(sets[(args.steps - 1) % nsets][2]) if args.dump_outputs and rank == 0 else None
 
     # ---- sustained: the same loop for about a second (power-capped clocks), same timing rules
     sustained = None
@@ -517,6 +549,9 @@ def main():
         }
         if world == 1:
             out["cpu_baseline"] = cpu_baseline(m, n, k, args.cpu_seconds, args.cpu_threads)
+        if dump is not None:
+            Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
+            np.save(Path(args.dump_outputs) / "c.npy", dump)
         print(json.dumps(out))
     if dist is not None:
         dist.barrier()

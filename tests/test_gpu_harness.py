@@ -80,6 +80,25 @@ def test_server_benchmark_cli_writes_result(base_dir):
     assert 20 <= rec["samples"] <= 600
 
 
+def test_bench_runs_the_requested_steps_and_dumps_reproducible_outputs(tmp_path):
+    """bench.py times exactly --steps launches, and --dump-outputs writes the same C for the same arguments."""
+    import numpy as np
+    m, n, k = 256, 512, 1024
+    dumps = []
+    for run in ("a", "b"):
+        cmd = [sys.executable, str(REPO / "bench.py"), "--mnk", f"{m}_{n}_{k}", "--steps", "7", "--warmup", "2",
+               "--sweep", "none", "--sustained_seconds", "0", "--e2e_steps", "1", "--cpu_seconds", "0.1",
+               "--dump-outputs", str(tmp_path / run)]
+        r = subprocess.run(cmd, cwd=REPO, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
+        d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert d["steps"] == 7 and d["gpu_launches"] == 7
+        c = np.load(tmp_path / run / "c.npy")
+        assert c.dtype == np.float32 and c.shape == (m, n) and np.isfinite(c).all() and c.std() > 1.0
+        dumps.append(c)
+    assert np.array_equal(dumps[0], dumps[1])
+
+
 def test_farm_harness_engine_runs_eval_one_file_for_a_shape(tmp_path):
     """farm_sweep.py --engine harness = the reference-style eval_one_file.sh per shape (0/1 check, one process per
     baseline, summary). Restricted to the cuBLASLt-auto-tuning pair, which is what the sweep's target needs."""

@@ -5,6 +5,7 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 
@@ -192,6 +193,27 @@ def test_bench_sweep_partition_covers_every_shape_once_and_balances():
         loads = [sum(bench.sweep_cost(s) for s in part) for part in parts]
         assert max(loads) <= 1.02 * (sum(loads) / world) + bench.sweep_cost((16384, 16384, 16384))
     assert bench.sweep_shapes("64_4096_64,4096_4096_4096") == [(64, 4096, 64), (4096, 4096, 4096)]
+
+
+def test_bench_rejects_a_step_count_below_one_and_a_dump_of_the_cpu_arm(tmp_path):
+    base = [sys.executable, str(REPO / "bench.py"), "--impl", "reference", "--mnk", "256_512_128", "--warmup", "1"]
+    r = subprocess.run(base + ["--steps", "0"], cwd=REPO, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 2 and "at least 1" in r.stderr
+    r = subprocess.run(base + ["--steps", "1", "--dump-outputs", str(tmp_path)], cwd=REPO, capture_output=True, text=True,
+                       timeout=300)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and not list(tmp_path.iterdir())
+
+
+def test_bench_output_sample_is_whole_or_a_fixed_subset():
+    import bench
+    small = torch.randn(64, 128).half()
+    got = bench.output_sample(small)
+    assert got.dtype == np.float32 and got.shape == (64, 128) and np.array_equal(got, small.float().numpy())
+    big = torch.arange(3000 * 3000, dtype=torch.float32).reshape(3000, 3000)       # each value is its flat index
+    got = bench.output_sample(big)
+    assert got.dtype == np.float32 and got.ndim == 1 and bench.DUMP_MAX_ELEMS // 2 < got.size <= bench.DUMP_MAX_ELEMS
+    assert (np.diff(got) > 0).all() and got[0] >= 0 and got[-1] < big.numel()      # sorted distinct positions
+    assert np.array_equal(bench.output_sample(big), got)                            # the same positions every time
 
 
 def test_bench_without_a_gpu_fails_loudly():
