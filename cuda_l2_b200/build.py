@@ -109,26 +109,6 @@ def build_trace(verbose: bool = False, force: bool = False) -> Path:
     return build_variant("trace", ["B200_HGEMM_TRACE"], verbose, force)
 
 
-def build_early_tma(verbose: bool = False, force: bool = False) -> Path:
-    """First TMA ring issued before the set-up barrier (-DB200_HGEMM_EARLY_TMA=1): the fixed-cost experiment."""
-    return build_variant("early", ["B200_HGEMM_EARLY_TMA=1"], verbose, force)
-
-
-def build_split_setup(verbose: bool = False, force: bool = False) -> Path:
-    """TMEM allocation behind the first set-up barrier, producer not waiting for it (-DB200_HGEMM_SPLIT_SETUP=1)."""
-    return build_variant("split", ["B200_HGEMM_SPLIT_SETUP=1"], verbose, force)
-
-
-def build_no_k_decomp(verbose: bool = False, force: bool = False) -> Path:
-    """Kernels without split-K / stream-K code (-DB200_HGEMM_NO_K_DECOMP=1): what does that code cost the plain path?"""
-    return build_variant("plain", ["B200_HGEMM_NO_K_DECOMP=1"], verbose, force)
-
-
-def build_wait_hint(ns: int = 2000, verbose: bool = False, force: bool = False) -> Path:
-    """mbarrier.try_wait with a suspend-time hint (-DB200_HGEMM_WAIT_HINT_NS): the polling-power experiment."""
-    return build_variant("hint", [f"B200_HGEMM_WAIT_HINT_NS={ns}"], verbose, force)
-
-
 def build_all(verbose: bool = False, force: bool = False) -> dict[str, Path]:
     out = {"capi": build_capi(verbose, force)}
     if (CSRC / "b200_baselines_capi.cu").exists():

@@ -230,8 +230,7 @@ int b200_hgemm_host(int acc_bits, const void* hA, const void* hB_kmajor, void* h
   // Blocks of >= 512 rows (a GEMM of fewer rows under-fills the device), at most kHostBlocks of them: the tail that
   // nothing overlaps — the last block's GEMM and copy out — shrinks with the block size.
   const int blocks = std::min(kHostBlocks, M / 512);
-  const bool pipelined = blocks >= 2 && (a_bytes + c_bytes) >= (size_t(8) << 20) &&
-                         !(std::getenv("B200_HGEMM_HOST_UNPIPELINED"));
+  const bool pipelined = blocks >= 2 && (a_bytes + c_bytes) >= (size_t(8) << 20);
   if (!pipelined) {
     if ((e = cudaMemcpyAsync(dA, hA, a_bytes, cudaMemcpyHostToDevice, 0)) != cudaSuccess) return int(e);
     if ((e = cudaMemcpyAsync(dB, hB_kmajor, b_bytes, cudaMemcpyHostToDevice, 0)) != cudaSuccess) return int(e);

@@ -107,17 +107,6 @@ __global__ void check_guard(const uint16_t* p, size_t n, uint16_t v, unsigned lo
   if (i < n && p[i] != v) atomicAdd(nbad, 1ull);
 }
 
-// probe: what do shared-memory addresses look like inside a 4-CTA cluster? (settles the pair-peer-bit convention)
-__global__ void __cluster_dims__(4, 1, 1) probe_cluster_addresses() {
-  __shared__ unsigned long long slot;
-  if (threadIdx.x == 0) {
-    unsigned rank, a = (unsigned)__cvta_generic_to_shared(&slot), m[4];
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
-    for (unsigned r = 0; r < 4; ++r) asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(m[r]) : "r"(a), "r"(r));
-    printf("PROBE rank %u cvta 0x%08x mapa[0..3] 0x%08x 0x%08x 0x%08x 0x%08x\n", rank, a, m[0], m[1], m[2], m[3]);
-  }
-}
-
 static inline dim3 g1(size_t n) { return dim3(unsigned((n + 255) / 256)); }
 
 struct Problem {
@@ -791,7 +780,6 @@ int main(int argc, char** argv) {
     return do_trace(atoi(argv[2]), atoi(argv[3]), atoi(argv[4]), atoi(argv[5]), atoi(argv[6]), argc > 7 ? atoi(argv[7]) : 0,
                     argc > 8 ? atoi(argv[8]) : 1, argc > 9 ? atoi(argv[9]) : 0);
 #endif
-  if (mode == "probe") { probe_cluster_addresses<<<4, 32>>>(); CK(cudaDeviceSynchronize()); return 0; }
   if (mode == "wall" && argc >= 6)
     return do_wall(atoi(argv[2]), atoi(argv[3]), atoi(argv[4]), atoi(argv[5]), argc > 6 ? atof(argv[6]) : 1.0,
                    argc > 7 ? atoi(argv[7]) : 0, argc > 8 ? atoi(argv[8]) : 0);

@@ -74,15 +74,8 @@ inline int encode_2d(CUtensorMap* map, const void* ptr, int rows, int cols, int 
   cuuint32_t estr[2] = {1, 1};
   // the swizzle span equals the box's inner extent: 64 fp16 = 128 B, 32 fp16 = 64 B
   const CUtensorMapSwizzle swz = box_cols == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-  // experiment hook: B200_HGEMM_L2_PROMOTION = 0 (none) | 1 (64 B) | 2 (128 B) | 3 (256 B, the default)
-  static const CUtensorMapL2promotion promo = [] {
-    const char* e = std::getenv("B200_HGEMM_L2_PROMOTION");
-    const int v = (e && e[0] >= '0' && e[0] <= '3') ? e[0] - '0' : 3;
-    return v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-         : v == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-  }();
   CUresult r = fn(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, swz, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? kOk : kEncodeFailed;
 }
 
@@ -301,12 +294,6 @@ int max_resident_clusters(const DeviceInfo& di) {
   return max_clusters;
 }
 
-// B200_HGEMM_NO_COOPERATIVE=1 launches the co-resident K-modes as ordinary grids (developer A/B of the launch cost).
-inline bool cooperative_enabled() {
-  static const bool on = [] { const char* e = std::getenv("B200_HGEMM_NO_COOPERATIVE"); return !(e && e[0] == '1'); }();
-  return on;
-}
-
 // B200_HGEMM_NO_PDL=1 launches without programmatic stream serialisation (developer A/B).
 inline bool pdl_enabled() {
   static const bool on = [] { const char* e = std::getenv("B200_HGEMM_NO_PDL"); return !(e && e[0] == '1'); }();
@@ -359,7 +346,7 @@ int launch_mode(const DeviceInfo& di, const LaunchArgs& a) {
   // grid starts only when all of it fits (other kernels holding SMs delay it instead of starving half of it into
   // the watchdog), and a grid that can never fit is refused with cudaErrorCooperativeLaunchTooLarge, which launch()
   // turns into the undivided schedule. (Cluster split-K needs nothing: a cluster is co-scheduled by the hardware.)
-  const bool coop = (KMODE == kWorkspaceSplitK || KMODE == kStreamK) && cooperative_enabled();
+  constexpr bool coop = (KMODE == kWorkspaceSplitK || KMODE == kStreamK);
   if (coop) {
     attr[na].id = cudaLaunchAttributeCooperative;
     attr[na].val.cooperative = 1;
@@ -368,26 +355,16 @@ int launch_mode(const DeviceInfo& di, const LaunchArgs& a) {
   // programmatic dependent launch: this kernel's prologue may overlap the tail of the stream's previous kernel; the
   // kernel itself waits (griddepcontrol.wait) before its first global-memory access. Back-to-back GEMMs lose the
   // 2-3 us of launch + set-up between them; a caller that synchronises after every call sees no difference.
-  // Together with the cooperative attribute only where the driver accepts the pair (B200_HGEMM_COOP_PDL=1 to try:
-  // the first refusal switches it off for the process).
-  static bool coop_pdl_ok = [] { const char* e = std::getenv("B200_HGEMM_COOP_PDL"); return e && e[0] == '1'; }();
-  const bool pdl = pdl_enabled() && (!coop || coop_pdl_ok);
-  if (pdl) {
+  // Not for a cooperative launch: the pair was measured to change nothing (DESIGN.md §6).
+  if (!coop && pdl_enabled()) {
     attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[na].val.programmaticStreamSerializationAllowed = 1;
     ++na;
   }
   cfg.attrs = attr;
   cfg.numAttrs = na;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, hgemm_tn_kernel<Cfg, KMODE>, a.ma, a.mb, a.mc, a.M, a.N, a.K, a.group_m,
-                                     a.plan.splits, a.plan.sk_tiles, a.ws, a.ctr, a.c, a.hint_a, a.hint_b);
-  if (e != cudaSuccess && coop && pdl && e != cudaErrorCooperativeLaunchTooLarge) {
-    cudaGetLastError();
-    coop_pdl_ok = false;               // the pair of attributes is not accepted here: cooperative only, from now on
-    cfg.numAttrs = na - 1;
-    e = cudaLaunchKernelEx(&cfg, hgemm_tn_kernel<Cfg, KMODE>, a.ma, a.mb, a.mc, a.M, a.N, a.K, a.group_m,
-                           a.plan.splits, a.plan.sk_tiles, a.ws, a.ctr, a.c, a.hint_a, a.hint_b);
-  }
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, hgemm_tn_kernel<Cfg, KMODE>, a.ma, a.mb, a.mc, a.M, a.N, a.K,
+                                           a.group_m, a.plan.splits, a.plan.sk_tiles, a.ws, a.ctr, a.c, a.hint_a, a.hint_b);
   return e == cudaSuccess ? kOk : int(e);
 }
 

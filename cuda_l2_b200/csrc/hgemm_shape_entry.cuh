@@ -11,15 +11,7 @@
                            : (SPLITS) > 1  ? (1u << b200::kWorkspaceSplitK)                              \
                            : (SPLITS) < -1 ? (1u << b200::kClusterSplitK) : 0u))
 
-#define B200_HGEMM_SHAPE_ENTRY(ACC_F32, BN, STAGES, CTA_GROUP, CLUSTER_M, CLUSTER_N, GROUP_M, SPLITS)                                       \
-  extern "C" int b200_hgemm_shape_entry(const void* A, const void* B_kmajor, void* C, int M, int N, int K,    \
-                                        void* stream) {                                                       \
-    return b200::host::launch<b200::Config<BN, STAGES, CTA_GROUP, ACC_F32, CLUSTER_M, CLUSTER_N>, B200_HGEMM_SHAPE_MODES(SPLITS)>(  \
-        A, B_kmajor, C, M, N, K, static_cast<cudaStream_t>(stream), GROUP_M, 0, SPLITS);                              \
-  }                                                                                                           \
-  extern "C" const char* b200_hgemm_shape_strerror(int status) { return b200::host::status_string(status); }
-
-// Same, for the configurations with 256 rows per CTA (M_REP = 2).
+// Exports the launcher of one configuration; M_REP = 2 for the configurations with 256 rows per CTA.
 #define B200_HGEMM_SHAPE_ENTRY_WIDE(ACC_F32, BN, STAGES, CTA_GROUP, CLUSTER_M, CLUSTER_N, M_REP, GROUP_M, SPLITS)            \
   extern "C" int b200_hgemm_shape_entry(const void* A, const void* B_kmajor, void* C, int M, int N, int K,    \
                                         void* stream) {                                                       \
@@ -27,3 +19,6 @@
         A, B_kmajor, C, M, N, K, static_cast<cudaStream_t>(stream), GROUP_M, 0, SPLITS);                      \
   }                                                                                                           \
   extern "C" const char* b200_hgemm_shape_strerror(int status) { return b200::host::status_string(status); }
+
+#define B200_HGEMM_SHAPE_ENTRY(ACC_F32, BN, STAGES, CTA_GROUP, CLUSTER_M, CLUSTER_N, GROUP_M, SPLITS) \
+  B200_HGEMM_SHAPE_ENTRY_WIDE(ACC_F32, BN, STAGES, CTA_GROUP, CLUSTER_M, CLUSTER_N, 1, GROUP_M, SPLITS)

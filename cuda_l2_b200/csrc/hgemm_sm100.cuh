@@ -52,16 +52,6 @@ constexpr int kAccStages = 2;        // TMEM accumulator ring depth
 // every launch — carries none of the three other epilogues: a quarter of the instructions, and registers to spare.
 enum KMode : int { kPlain = 0, kWorkspaceSplitK = 1, kClusterSplitK = 2, kStreamK = 3 };
 
-#ifndef B200_HGEMM_NO_K_DECOMP
-#define B200_HGEMM_NO_K_DECOMP 0     // experiment: kernels without split-K / stream-K code
-#endif
-#ifndef B200_HGEMM_SPLIT_SETUP
-#define B200_HGEMM_SPLIT_SETUP 0     // experiment: TMEM allocation after the barrier-publishing barrier, producer not waiting for it
-#endif
-#ifndef B200_HGEMM_EARLY_TMA
-#define B200_HGEMM_EARLY_TMA 0       // experiment: first loads before the set-up barrier (see the set-up block)
-#endif
-
 // Developer instrumentation (only in builds with -DB200_HGEMM_TRACE, i.e. libb200_hgemm_trace.so; the product build
 // contains none of it): per-CTA timestamps of the kernel's phases, read back by `dev_check_trace trace`.
 //   slot 0 entry | 1 setup done | 2 first TMA issued | 3 last TMA issued | 4 first stage landed (MMA warp)
@@ -129,10 +119,9 @@ struct Config {
   static constexpr int EPI_GROUPS = EPI_CHUNKS >= 2 ? 2 : 1;
   static constexpr int EPI_CHUNKS_PER_GROUP = (EPI_CHUNKS + EPI_GROUPS - 1) / EPI_GROUPS;
   static constexpr int NUM_THREADS = EPI_GROUPS == 2 ? kNumThreads : kNumThreads - 128;   // no warps that would only wait
-  // which K-decompositions this configuration's kernel carries (B200_HGEMM_NO_K_DECOMP: an experiment build without
-  // any of them, to see what their code costs the plain path)
-  static constexpr bool SPLIT_K = !B200_HGEMM_NO_K_DECOMP && CTA_GROUP_ * CLUSTER_M_ * CLUSTER_N_ == 1 && BN_ >= 64 && M_REP_ == 1;
-  static constexpr bool STREAM_K = !B200_HGEMM_NO_K_DECOMP && CLUSTER_M_ * CLUSTER_N_ == 1 && BN_ >= 64 && M_REP_ == 1;
+  // which K-decompositions this configuration's kernel can be instantiated with
+  static constexpr bool SPLIT_K = CTA_GROUP_ * CLUSTER_M_ * CLUSTER_N_ == 1 && BN_ >= 64 && M_REP_ == 1;
+  static constexpr bool STREAM_K = CLUSTER_M_ * CLUSTER_N_ == 1 && BN_ >= 64 && M_REP_ == 1;
   static constexpr int EPI_BUF_BYTES = 32 * EPI_N * 2;       // one warp, one chunk: 32 rows x EPI_N fp16
   static constexpr int EPI_BYTES = 8 * 32 * 64 * 2;          // 8 warps x one staging buffer (sized for EPI_N = 64)
   static constexpr int BAR_BYTES = 512;
@@ -179,6 +168,38 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
 
 constexpr int kMaxSplitTiles = 256;   // split-K is only used when tiles * splits <= #SMs
 
+// TMEM columns [32j, 32j + 32) of this warp's lanes as fp32, whatever the accumulator type
+template <class Cfg>
+__device__ __forceinline__ void tmem_load_f32_x32(uint32_t taddr0, int j, float (&f)[32]) {
+  using namespace ptx;
+  uint32_t v[32];
+  if constexpr (Cfg::ACC_F32) {
+    tmem_ld_32x32b_x32(taddr0 + j * 32, v);
+    tmem_ld_wait();
+#pragma unroll
+    for (int i = 0; i < 32; ++i) f[i] = __uint_as_float(v[i]);
+  } else {
+    // fp16 accumulators: 64 columns arrive packed two per register, so 32 columns fill half of the registers
+    tmem_ld_32x32b_x32_pack16(taddr0 + (j / 2) * 64, v);
+    tmem_ld_wait();
+#pragma unroll
+    for (int i = 0; i < 16; ++i) {
+      const __half2 h = *reinterpret_cast<const __half2*>(&v[(j & 1) * 16 + i]);
+      f[2 * i] = __low2float(h);
+      f[2 * i + 1] = __high2float(h);
+    }
+  }
+}
+
+// Four adjacent output columns rounded once and stored to C (the split-K reductions' direct stores)
+template <class Cfg>
+__device__ __forceinline__ void store_out_x4(__half* __restrict__ C, int gm, int gn, int N, float4 acc) {
+  uint2 out;
+  out.x = ptx::pack_out_x2_rn<Cfg::BF16>(acc.x, acc.y);
+  out.y = ptx::pack_out_x2_rn<Cfg::BF16>(acc.z, acc.w);
+  *reinterpret_cast<uint2*>(C + size_t(gm) * N + gn) = out;
+}
+
 // Split-K epilogue (CTA_GROUP == 1, one (tile, split) unit per CTA, all units resident at once).
 //   phase 1  every split writes its 128 x BN fp32 partial tile to the workspace slot (tile, split);
 //   barrier  a per-tile arrival counter in global memory (release/acquire at gpu scope);
@@ -197,24 +218,7 @@ __device__ __forceinline__ void splitk_epilogue(uint32_t taddr0, int q, int lane
 #pragma unroll
   for (int j = 0; j < BN / 32; ++j) {
     float f[32];
-    if constexpr (Cfg::ACC_F32) {
-      uint32_t v[32];
-      tmem_ld_32x32b_x32(taddr0 + j * 32, v);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 32; ++i) f[i] = __uint_as_float(v[i]);
-    } else {
-      // fp16 accumulators: 32 columns arrive packed two per register in the first 16 registers
-      uint32_t v[32];
-      tmem_ld_32x32b_x32_pack16(taddr0 + (j / 2) * 64, v);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const __half2 h = *reinterpret_cast<const __half2*>(&v[(j & 1) * 16 + i]);
-        f[2 * i] = __low2float(h);
-        f[2 * i + 1] = __high2float(h);
-      }
-    }
+    tmem_load_f32_x32<Cfg>(taddr0, j, f);
 #pragma unroll
     for (int i = 0; i < 8; ++i)
       __stcg(reinterpret_cast<float4*>(slot + j * 32) + i, make_float4(f[4 * i], f[4 * i + 1], f[4 * i + 2], f[4 * i + 3]));
@@ -260,10 +264,7 @@ __device__ __forceinline__ void splitk_epilogue(uint32_t taddr0, int q, int lane
         const float4 p = ld_shared_v4f(red_smem + uint32_t(sp) * slice_bytes + uint32_t(i) * 16u);
         acc.x += p.x; acc.y += p.y; acc.z += p.z; acc.w += p.w;
       }
-      uint2 out;
-      out.x = pack_out_x2_rn<Cfg::BF16>(acc.x, acc.y);
-      out.y = pack_out_x2_rn<Cfg::BF16>(acc.z, acc.w);
-      *reinterpret_cast<uint2*>(C + size_t(gm) * N + gn) = out;
+      store_out_x4<Cfg>(C, gm, gn, N, acc);
     }
   }
   asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -292,23 +293,7 @@ __device__ __forceinline__ void cluster_splitk_park(uint32_t taddr0, int q, int 
 #pragma unroll
   for (int j = 0; j < BN / 32; ++j) {
     float f[32];
-    if constexpr (Cfg::ACC_F32) {
-      uint32_t v[32];
-      tmem_ld_32x32b_x32(taddr0 + j * 32, v);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 32; ++i) f[i] = __uint_as_float(v[i]);
-    } else {
-      uint32_t v[32];
-      tmem_ld_32x32b_x32_pack16(taddr0 + (j / 2) * 64, v);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const __half2 h = *reinterpret_cast<const __half2*>(&v[(j & 1) * 16 + i]);
-        f[2 * i] = __low2float(h);
-        f[2 * i + 1] = __high2float(h);
-      }
-    }
+    tmem_load_f32_x32<Cfg>(taddr0, j, f);
 #pragma unroll
     for (int i = 0; i < 8; ++i)
       st_shared_v4f(row_addr + uint32_t(j) * 128u + uint32_t(i) * 16u, f[4 * i], f[4 * i + 1], f[4 * i + 2], f[4 * i + 3]);
@@ -339,10 +324,7 @@ __device__ __forceinline__ void cluster_splitk_reduce(int e, int split, int spli
         acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
       }
     }
-    uint2 out;
-    out.x = pack_out_x2_rn<Cfg::BF16>(acc.x, acc.y);
-    out.y = pack_out_x2_rn<Cfg::BF16>(acc.z, acc.w);
-    *reinterpret_cast<uint2*>(C + size_t(gm) * N + gn) = out;
+    store_out_x4<Cfg>(C, gm, gn, N, acc);
   }
 }
 
@@ -355,7 +337,6 @@ __device__ __forceinline__ void cluster_splitk_reduce(int e, int split, int spli
 // warps stay as decoupled as in the plain epilogue and the flags are zero again when the grid ends.
 constexpr int kMaxStreamKSlots = 160;   // CTAs of a launch (>= 148 SMs), one partial-tile slot each
 constexpr int kStreamKFlagsPerSlot = 8; // epilogue warps
-constexpr bool kStreamKBulkFixup = true;   // false: always fetch the partials with register loads (streamk_own)
 
 template <class Cfg>
 struct StreamK {
@@ -366,6 +347,10 @@ struct StreamK {
   static constexpr size_t SLOT_BYTES = size_t(SLOT_U4) * 16;
   static constexpr uint32_t CHUNK_BYTES = uint32_t(CHUNK_U4) * 16;
   static constexpr int FIX_RING = Cfg::FIX_REGION_BYTES / int(CHUNK_BYTES) >= 3 ? 3 : Cfg::FIX_REGION_BYTES / int(CHUNK_BYTES);
+  // The owner adds its own accumulator to the summed partials in pieces of PIECE columns, so that (sums + values in
+  // flight + own accumulator) stays near the register footprint of the plain epilogue: fp32 images in two pieces of 32
+  // columns, fp16 images (half the registers) in one piece of 64.
+  static constexpr int PIECE = Cfg::ACC_F32 ? 32 : 64;
 };
 
 // this warp's chunk `j` of the accumulator, raw: fp32 bit patterns, or fp16 pairs (two columns per register)
@@ -436,17 +421,10 @@ __device__ __forceinline__ void streamk_contribute(const EpilogueWarp& w, uint32
   if (w.lane == 0) st_release_gpu(flags + slot * kStreamKFlagsPerSlot + w.ew, 1u);
 }
 
-// Owner: the partials of `n` contributors (slots slot0, slot0 + slot_stride, ... — increasing k) summed in fp32 in that
-// fixed order, plus the own accumulator, rounded once, stored like any other tile. The partials were written long
-// before (they are their workers' first units), so the first chunk's are fetched BEFORE waiting for the own
-// accumulator (`wait_acc`): their L2 latency hides behind the tail of the main loop.
-template <class Cfg, class WaitAcc, class ReleaseTmem>
-__device__ __forceinline__ void streamk_own(const EpilogueWarp& w, uint32_t taddr0, const uint4* __restrict__ ws,
-                                            unsigned* __restrict__ flags, int slot0, int slot_stride, int n,
-                                            const CUtensorMap* tmap_c, int m0, int n0, int M, int N,
-                                            WaitAcc wait_acc, ReleaseTmem release_tmem) {
+// Owner, before it reads any partial: lane 0 waits until each of the `n` contributors has raised this warp's flag.
+__device__ __forceinline__ void streamk_wait_contributors(const EpilogueWarp& w, const unsigned* __restrict__ flags,
+                                                          int slot0, int slot_stride, int n) {
   using namespace ptx;
-  using SK = StreamK<Cfg>;
   if (w.lane == 0) {
     for (int p = 0; p < n; ++p) {
       const unsigned* f = flags + (slot0 + p * slot_stride) * kStreamKFlagsPerSlot + w.ew;
@@ -458,11 +436,57 @@ __device__ __forceinline__ void streamk_own(const EpilogueWarp& w, uint32_t tadd
     }
   }
   __syncwarp();
+}
+
+// Owner, done: lower the flags again. This warp is their only reader, and the next writer is a later launch.
+__device__ __forceinline__ void streamk_lower_flags(const EpilogueWarp& w, unsigned* __restrict__ flags, int slot0,
+                                                    int slot_stride, int n) {
+  __syncwarp();
+  if (w.lane == 0)
+    for (int p = 0; p < n; ++p) flags[(slot0 + p * slot_stride) * kStreamKFlagsPerSlot + w.ew] = 0u;
+}
+
+// Owner: piece `h` (StreamK::PIECE columns) of the chunk at `taddr_chunk`: the own accumulator added to the summed
+// partials `f` of that piece, rounded once and packed into its place in `packed`. `last`: the warp's last TMEM read,
+// after which the accumulator stage goes back to the MMA warp.
+template <class Cfg, class ReleaseTmem>
+__device__ __forceinline__ void streamk_add_own(uint32_t taddr_chunk, int h, const float* f,
+                                                uint32_t (&packed)[Cfg::EPI_N / 2], bool last, ReleaseTmem release_tmem) {
+  using namespace ptx;
+  if constexpr (Cfg::ACC_F32) {
+    uint32_t v[32];
+    tmem_ld_32x32b_x32(taddr_chunk + 32 * h, v);
+    tmem_ld_wait();
+    if (last) release_tmem();
+#pragma unroll
+    for (int i = 0; i < 16; ++i)
+      packed[16 * h + i] = pack_out_x2_rn<Cfg::BF16>(f[2 * i] + __uint_as_float(v[2 * i]), f[2 * i + 1] + __uint_as_float(v[2 * i + 1]));
+  } else {
+    uint32_t r[StreamK<Cfg>::REGS];
+    streamk_load_chunk<Cfg>(taddr_chunk, r);
+    if (last) release_tmem();
+#pragma unroll
+    for (int i = 0; i < Cfg::EPI_N / 2; ++i) {
+      const __half2 hh = *reinterpret_cast<const __half2*>(&r[i]);
+      packed[i] = pack_out_x2_rn<Cfg::BF16>(f[2 * i] + __low2float(hh), f[2 * i + 1] + __high2float(hh));
+    }
+  }
+}
+
+// Owner: the partials of `n` contributors (slots slot0, slot0 + slot_stride, ... — increasing k) summed in fp32 in that
+// fixed order, plus the own accumulator, rounded once, stored like any other tile. The partials were written long
+// before (they are their workers' first units), so the first chunk's are fetched BEFORE waiting for the own
+// accumulator (`wait_acc`): their L2 latency hides behind the tail of the main loop.
+template <class Cfg, class WaitAcc, class ReleaseTmem>
+__device__ __forceinline__ void streamk_own(const EpilogueWarp& w, uint32_t taddr0, const uint4* __restrict__ ws,
+                                            unsigned* __restrict__ flags, int slot0, int slot_stride, int n,
+                                            const CUtensorMap* tmap_c, int m0, int n0, int M, int N,
+                                            WaitAcc wait_acc, ReleaseTmem release_tmem) {
+  using namespace ptx;
+  using SK = StreamK<Cfg>;
+  streamk_wait_contributors(w, flags, slot0, slot_stride, n);
   const size_t warp_off = size_t(w.q * Cfg::EPI_CHUNKS) * SK::CHUNK_U4 + w.lane;
-  // A chunk is summed in pieces of kPiece columns so that (sums + values in flight + own accumulator) stays near the
-  // register footprint of the plain epilogue: fp32 images in two pieces of 32 columns, fp16 images (half the
-  // registers) in one piece of 64.
-  constexpr int kPiece = Cfg::ACC_F32 ? 32 : 64;                  // columns
+  constexpr int kPiece = SK::PIECE;                               // columns
   constexpr int kPieceQuads = SK::R4 * kPiece / Cfg::EPI_N;       // image quads per piece (8 in both cases)
   constexpr int kBatch = 4;                                       // quads in flight per lane
 #pragma unroll 1
@@ -500,31 +524,11 @@ __device__ __forceinline__ void streamk_own(const EpilogueWarp& w, uint32_t tadd
       }
       if (j == w.j_begin && h == 0) wait_acc();
       const bool last = (j == w.j_end - 1) && (h == Cfg::EPI_N / kPiece - 1);
-      if constexpr (Cfg::ACC_F32) {
-        uint32_t v[32];
-        tmem_ld_32x32b_x32(taddr0 + j * Cfg::EPI_N + 32 * h, v);
-        tmem_ld_wait();
-        if (last) release_tmem();
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          packed[16 * h + i] = pack_out_x2_rn<Cfg::BF16>(f[2 * i] + __uint_as_float(v[2 * i]), f[2 * i + 1] + __uint_as_float(v[2 * i + 1]));
-      } else {
-        uint32_t r[SK::REGS];
-        streamk_load_chunk<Cfg>(taddr0 + j * Cfg::EPI_N, r);
-        if (last) release_tmem();
-#pragma unroll
-        for (int i = 0; i < Cfg::EPI_N / 2; ++i) {
-          const __half2 hh = *reinterpret_cast<const __half2*>(&r[i]);
-          packed[i] = pack_out_x2_rn<Cfg::BF16>(f[2 * i] + __low2float(hh), f[2 * i + 1] + __high2float(hh));
-        }
-      }
+      streamk_add_own<Cfg>(taddr0 + j * Cfg::EPI_N, h, f, packed, last, release_tmem);
     }
     epilogue_store_chunk<Cfg>(packed, w.epi_buf, w.row_off, w.sw, w.lane, tmap_c, n0 + j * Cfg::EPI_N, m0, M, N);
   }
-  // lower the flags again: this warp is their only reader, and the next writer is a later launch
-  __syncwarp();
-  if (w.lane == 0)
-    for (int p = 0; p < n; ++p) flags[(slot0 + p * slot_stride) * kStreamKFlagsPerSlot + w.ew] = 0u;
+  streamk_lower_flags(w, flags, slot0, slot_stride, n);
 }
 
 // Owner whose unit ends the worker's schedule: nothing hides the fix-up any more, and register loads would crawl
@@ -542,17 +546,7 @@ __device__ __forceinline__ void streamk_own_bulk(const EpilogueWarp& w, uint32_t
   using SK = StreamK<Cfg>;
   constexpr int RING = SK::FIX_RING;
   static_assert(RING >= 2, "the fix-up ring needs two chunk images per epilogue warp");
-  if (w.lane == 0) {
-    for (int p = 0; p < n; ++p) {
-      const unsigned* f = flags + (slot0 + p * slot_stride) * kStreamKFlagsPerSlot + w.ew;
-      unsigned spins = 0;
-      while (ld_acquire_gpu(f) == 0u) {
-        __nanosleep(64);
-        if (++spins > (1u << 24)) { printf("b200_hgemm watchdog: stream-K slot %d never arrived\n", slot0 + p * slot_stride); __trap(); }
-      }
-    }
-  }
-  __syncwarp();
+  streamk_wait_contributors(w, flags, slot0, slot_stride, n);
   const int total = (w.j_end - w.j_begin) * n;   // items in (chunk, contributor) order
   auto issue = [&](int i) {
     if (w.lane == 0) {
@@ -598,34 +592,14 @@ __device__ __forceinline__ void streamk_own_bulk(const EpilogueWarp& w, uint32_t
       }
     }
     uint32_t packed[Cfg::EPI_N / 2];
-    const bool last = (j == w.j_end - 1);
-    if constexpr (Cfg::ACC_F32) {
 #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        uint32_t v[32];
-        tmem_ld_32x32b_x32(taddr0 + j * Cfg::EPI_N + 32 * h, v);
-        tmem_ld_wait();
-        if (last && h == 1) release_tmem();
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          packed[16 * h + i] = pack_out_x2_rn<Cfg::BF16>(f[32 * h + 2 * i] + __uint_as_float(v[2 * i]),
-                                             f[32 * h + 2 * i + 1] + __uint_as_float(v[2 * i + 1]));
-      }
-    } else {
-      uint32_t r[SK::REGS];
-      streamk_load_chunk<Cfg>(taddr0 + j * Cfg::EPI_N, r);
-      if (last) release_tmem();
-#pragma unroll
-      for (int i = 0; i < Cfg::EPI_N / 2; ++i) {
-        const __half2 hh = *reinterpret_cast<const __half2*>(&r[i]);
-        packed[i] = pack_out_x2_rn<Cfg::BF16>(f[2 * i] + __low2float(hh), f[2 * i + 1] + __high2float(hh));
-      }
+    for (int h = 0; h < Cfg::EPI_N / SK::PIECE; ++h) {
+      const bool last = (j == w.j_end - 1) && (h == Cfg::EPI_N / SK::PIECE - 1);
+      streamk_add_own<Cfg>(taddr0 + j * Cfg::EPI_N, h, f + h * SK::PIECE, packed, last, release_tmem);
     }
     epilogue_store_chunk<Cfg>(packed, w.epi_buf, w.row_off, w.sw, w.lane, tmap_c, n0 + j * Cfg::EPI_N, m0, M, N);
   }
-  __syncwarp();
-  if (w.lane == 0)
-    for (int p = 0; p < n; ++p) flags[(slot0 + p * slot_stride) * kStreamKFlagsPerSlot + w.ew] = 0u;
+  streamk_lower_flags(w, flags, slot0, slot_stride, n);
 }
 
 template <class Cfg, int KMODE = kPlain>
@@ -713,47 +687,7 @@ hgemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,   // A  [M,K]  box {
     tma_prefetch_desc(&tmap_a);
     tma_prefetch_desc(&tmap_b);
     tma_prefetch_desc(&tmap_c);
-#if B200_HGEMM_EARLY_TMA
-    // Experiment (default off): a CTA that shares its barriers with nobody need not wait for the set-up barrier (and
-    // the TMEM allocation behind it) before its first loads leave — the first ring of the first unit is issued here,
-    // by the thread that has just initialised the barriers; the producer loop below starts behind it.
-    if constexpr (Cfg::CLUSTER_CTAS == 1) {
-      WorkIter first_work(worker, num_workers, num_tiles, num_k_blocks, splits, sk_tiles);
-      WorkUnit u0;
-      if (first_work.next(u0)) {
-        fence_proxy_async_smem();   // the initialised barriers (generic proxy) before the loads' complete_tx (async proxy)
-        const TileCoord tc = tile_coord(u0.tile, num_m_blocks, num_n_blocks, group_m);
-        const int npre = min(STAGES, u0.kb1 - u0.kb0);
-        for (int st = 0; st < npre; ++st) {
-          mbar_arrive_expect_tx(bar_full + 8 * st, Cfg::STAGE_BYTES);
-          tma_load_2d_hint<1>(smem_a + st * Cfg::A_STAGE_BYTES, &tmap_a, bar_full + 8 * st, (u0.kb0 + st) * kBlockK,
-                              tc.m_blk * Cfg::TILE_M, hint_a);
-          tma_load_2d_hint<1>(smem_b + st * Cfg::B_STAGE_BYTES, &tmap_b, bar_full + 8 * st, (u0.kb0 + st) * kBlockK,
-                              tc.n_blk * BN, hint_b);
-        }
-      }
-    }
-#endif
   }
-#if B200_HGEMM_SPLIT_SETUP
-  // Experiment (default off): the barrier that publishes the initialised mbarriers comes first, the TMEM allocation
-  // after it, published by a second barrier that the producer warp does not take part in — its first loads are in
-  // flight while the allocator works.
-  __syncwarp();
-  if constexpr (Cfg::CLUSTER_CTAS > 1) cluster_sync_all(); else __syncthreads();
-  uint32_t tmem_base = 0;
-  if (warp != 0) {
-    if (warp == 2) {
-      tmem_alloc<CG>(tmem_slot, Cfg::TMEM_COLS);
-      tmem_relinquish<CG>();
-    }
-    __syncwarp();
-    tc_fence_before_sync();
-    asm volatile("bar.sync 2, %0;" ::"n"(Cfg::NUM_THREADS - 32) : "memory");
-    tc_fence_after_sync();
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  }
-#else
   if (warp == 2) {
     tmem_alloc<CG>(tmem_slot, Cfg::TMEM_COLS);
     tmem_relinquish<CG>();
@@ -764,7 +698,6 @@ hgemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,   // A  [M,K]  box {
   tc_fence_after_sync();
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-#endif
   B200_TRACE_ONLY(if (threadIdx.x == 64) B200_TRACE(1);)
 
   // Programmatic dependent launch (the host sets cudaLaunchAttributeProgrammaticStreamSerialization): this grid may have
@@ -799,24 +732,11 @@ hgemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,   // A  [M,K]  box {
     B200_TRACE_ONLY(bool trace_first = true;)
     WorkIter work(worker, num_workers, num_tiles, num_k_blocks, splits, sk_tiles);
     WorkUnit u;
-#if B200_HGEMM_EARLY_TMA
-    bool skip_issued = (Cfg::CLUSTER_CTAS == 1);   // the first ring of the first unit left during set-up
-#endif
     while (work.next(u)) {
       const TileCoord tc = tile_coord(u.tile, num_m_blocks, num_n_blocks, group_m);
       const int m0 = (tc.m_blk * CM + cm) * Cfg::TILE_M + int(cta_rank) * Cfg::CTA_M + cn * Cfg::A_BOX_ROWS;
       const int n0 = (tc.n_blk * CN + cn) * BN + int(cta_rank) * Cfg::LOAD_N + cm * Cfg::B_BOX_ROWS;
-      int kb_begin = u.kb0;
-#if B200_HGEMM_EARLY_TMA
-      if (skip_issued) {
-        const int npre = min(STAGES, u.kb1 - u.kb0);
-        kb_begin += npre;
-        stage = npre % STAGES;
-        phase = uint32_t(npre / STAGES);
-        skip_issued = false;
-      }
-#endif
-      for (int kb = kb_begin; kb < u.kb1; ++kb) {
+      for (int kb = u.kb0; kb < u.kb1; ++kb) {
         mbar_wait(bar_empty + 8 * stage, phase ^ 1);
         if (elect_one()) {
           if (is_leader) mbar_arrive_expect_tx(bar_full + 8 * stage, Cfg::STAGE_BYTES * CG);
@@ -945,7 +865,7 @@ hgemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a,   // A  [M,K]  box {
       if constexpr (KMODE == kStreamK) {
         if (u.kb0 == 0 && u.kb1 < num_k_blocks) {   // the head of a tile, which owns it
           const int n = streamk_contributors(worker, num_workers, sk_tiles * num_k_blocks, t, num_k_blocks);
-          if (kStreamKBulkFixup && !work.has_more())   // nothing left to hide the fix-up behind: stream it through shared memory
+          if (!work.has_more())   // nothing left to hide the fix-up behind: stream it through shared memory
             streamk_own_bulk<Cfg>(ew, taddr_acc, ws4, sk_flags, (worker + 1) * CG + int(cta_rank), CG, n, &tmap_c,
                                   m_tile0 + q * 32, n0, M, N, smem_a + uint32_t(ew.ew) * Cfg::FIX_REGION_BYTES,
                                   bar_fix + 8 * 3 * ew.ew, wait_acc, release_tmem);

@@ -64,23 +64,8 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t byt
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes)
                : "memory");
 }
-// B200_HGEMM_WAIT_HINT_NS (experiment, default off): upper bound in ns the hardware may keep a waiting thread suspended
-// before try_wait returns false; a completed phase wakes it at once either way, so a large hint only thins out
-// the polling of warps that wait for most of the kernel (the epilogue warps during a long main loop).
-#ifndef B200_HGEMM_WAIT_HINT_NS
-#define B200_HGEMM_WAIT_HINT_NS 0
-#endif
 __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
   uint32_t ok;
-#if B200_HGEMM_WAIT_HINT_NS > 0
-  asm volatile(
-      "{\n\t.reg .pred P;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, P;\n\t}\n"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity), "r"(uint32_t(B200_HGEMM_WAIT_HINT_NS))
-      : "memory");
-#else
   asm volatile(
       "{\n\t.reg .pred P;\n\t"
       "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
@@ -88,7 +73,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
       : "=r"(ok)
       : "r"(bar), "r"(parity)
       : "memory");
-#endif
   return ok != 0;
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
